@@ -54,7 +54,16 @@ def parse():
                     help="N>1: 1 = expert parameters FSDP-sharded over the ranks (fp32 master shards, cast+push all-gather with "
                          "prefetch, re-gather in backward, reduce-scatter of the gradients: xtuner_b200/fsdp_experts.py) inside "
                          "the timed step; 0 = independent replicas (no inter-rank traffic); -1 = 1 when N>1")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed (loss, output of the last layer, "
+                         "gradient of the step input, every parameter gradient) as DIR/<name>.npy in float32; arrays larger "
+                         "than an equal share of 64 MB are replaced by a fixed seeded sample of their elements")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
+    return args
 
 
 # ----------------------------------------------------------------------------------------------------
@@ -425,6 +434,29 @@ def gpu_reference_record(kernel_us, ms_step, L):
             "side_by_side": side}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes ``arrays`` (name -> tensor) as ``out_dir/<name>.npy`` in float32, at most ``DUMP_BYTES`` in all: an array
+    larger than its equal share keeps that many elements, at positions drawn by a generator seeded with the array's size, so
+    two runs with the same arguments store the same elements."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // 4 // max(1, len(arrays))
+    picks = {}  # numel -> sampled positions
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > share:
+            if t.numel() not in picks:
+                g = torch.Generator().manual_seed(t.numel())
+                picks[t.numel()] = torch.randperm(t.numel(), generator=g)[:share].sort().values.to(t.device)
+            t = t.reshape(-1)[picks[t.numel()]]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 def default_parallelism(world, fsdp_flag):
     return f"fsdp={world} (ep=1)" if (world > 1 and fsdp_flag != 0) else f"dp{world} (ep=1)"
 
@@ -733,10 +765,17 @@ def run_ours(args):
         e.record()
         prof.append((fn_name, s, e))
 
+    last: dict = {}  # --dump-outputs: the tensors the most recent step() returned or wrote (in graph mode: the graph's own)
+
+    def keep(loss, h, x_leaf):
+        if args.dump_outputs:
+            last.clear()
+            last.update(loss=loss.detach(), output=h.detach(), input_grad=x_leaf.grad, grads=[p.grad for p in params])
+
     def step(x_in):
         for p in params:
             p.grad = None
-        h = x_in.detach().requires_grad_(True)
+        h = x_leaf = x_in.detach().requires_grad_(True)
         if use_fsdp:
             eng.begin_step()  # all-gather (cast + push) of layer 0 on the exchange stream
             for i in range(L):
@@ -746,6 +785,7 @@ def run_ours(args):
             loss = h.float().square().mean()
             loss.backward()
             eng.end_step()  # the compute stream joins the last reduce-scatter; .grad = averaged fp32 shard gradients
+            keep(loss, h, x_leaf)
             return loss
         for m in layers:
             # MoE half of the decoder layer: residual = h; x = post_attention_layernorm(h); h = moe(x) + residual
@@ -753,6 +793,7 @@ def run_ours(args):
             h, _ = m(h) if args.path == "block" else m(norm(h), h)
         loss = h.float().square().mean()
         loss.backward()
+        keep(loss, h, x_leaf)
         return loss
 
     norm_w = torch.ones(H, dtype=torch.bfloat16, device=dev)
@@ -796,7 +837,7 @@ def run_ours(args):
 
     # ---- optional CUDA-graph capture of the whole step (no host syncs on the path, so it is capturable) ----
     mode = "eager"
-    graph = None
+    graph = graph_outputs = None
     static_x = x_dev.clone()
     static_loss = None
     side = torch.cuda.Stream()
@@ -820,6 +861,7 @@ def run_ours(args):
     if args.mode == "graph":
         try:
             graph, static_loss = capture()
+            graph_outputs = dict(last)  # the captured step's tensors: every replay rewrites them in place
             mode = "cuda_graph"
         except Exception as ex:  # noqa: BLE001
             sys.stderr.write(f"[bench] CUDA graph capture failed ({type(ex).__name__}: {ex}); falling back to eager\n")
@@ -889,6 +931,17 @@ def run_ours(args):
     sampler.end()
     clocks = sampler.stop()
     ms_e2e = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        out = graph_outputs if graph is not None else last
+        if use_fsdp:
+            names = ([f"layer{i:02d}.experts.fused_w1w3.weight_shard" for i in range(L)]
+                     + [f"layer{i:02d}.experts.fused_w2.weight_shard" for i in range(L)]
+                     + [f"layer{i:02d}.{n}" for i in range(L) for n in ("post_attention_layernorm.weight", "gate.weight")])
+        else:
+            names = [f"layer{i:02d}.{n}" for i, m in enumerate(layers) for n, _ in m.named_parameters()]
+        arrays = {"loss": out["loss"], "output": out["output"], "input_grad": out["input_grad"]}
+        arrays.update({n + ".grad": g for n, g in zip(names, out["grads"], strict=True) if g is not None})
+        dump_outputs(args.dump_outputs, arrays)
 
     # ---- N>1: the same step with the exchange switched off (stream/event choreography kept, no barrier/push/pull) ->
     # exposed exchange time; then the exchange kernels alone -> NVLink roofline ---------------------------------

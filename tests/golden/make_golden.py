@@ -450,8 +450,80 @@ def gen_fp8():
                            x_scales=xs))
 
 
+# ---------------------------------------------------------------------------------------------
+# 8. the reference's seams the plugin plugs into: signatures, result keys, state-dict layout, module globals the
+#    plugin rebinds, and what the fp8 cast functions return (tests/test_dropin_conformance.py,
+#    tests/test_plugin_reference_cpu.py)
+# ---------------------------------------------------------------------------------------------
+def _params(fn):
+    import inspect
+
+    return [(n, int(p.kind), p.default is not inspect.Parameter.empty) for n, p in inspect.signature(fn).parameters.items()
+            if n != "self"]
+
+
+def _sha256(t: torch.Tensor) -> str:
+    import hashlib
+
+    return hashlib.sha256(t.contiguous().view(torch.uint8).numpy().tobytes()).hexdigest()
+
+
+def gen_seams():
+    import inspect
+
+    import xtuner.v1.float8.fsdp_utils as fu
+    import xtuner.v1.module.attention.mha as mha
+    import xtuner.v1.module.grouped_linear.moe_group_linear as mgl
+    from xtuner.v1.module.dispatcher.base import GenericDispatcher
+    from xtuner.v1.module.router.noaux_router import NoAuxRouter as RefNoAux
+    from xtuner.v1.module.router.protocol import RouterResults
+    from xtuner.v1.ops.comm.all_to_all import ulysses_all_to_all as ref_a2a
+    from xtuner.v1.ops.moe.protocol import GroupGemmProtocol, MoePermuteProtocol, MoeUnpermuteProtocol
+
+    def positional(fn):
+        return [n for n, p in inspect.signature(fn).parameters.items() if n != "self" and p.kind != inspect.Parameter.KEYWORD_ONLY]
+
+    abstract = sorted(GenericDispatcher.__abstractmethods__)
+    out = dict(
+        dispatcher_abstract=abstract,
+        dispatcher_params={name: _params(getattr(NaiveDispatcher, name)) for name in abstract},
+        dispatcher_init=_params(NaiveDispatcher.__init__),
+        protocol_positional=dict(group_gemm=positional(GroupGemmProtocol.__call__), permute=positional(MoePermuteProtocol.__call__),
+                                 unpermute=positional(MoeUnpermuteProtocol.__call__)),
+        router_results_keys=sorted(RouterResults.__annotations__),
+        greedy_router_init=_params(GreedyRouter.__init__),
+        noaux_router_init=_params(RefNoAux.__init__),
+        greedy_router_forward=_params(GreedyRouter.forward),
+        ulysses_all_to_all=list(inspect.signature(ref_a2a).parameters),
+        module_globals={"xtuner.v1.module.attention.mha": ["ulysses_all_to_all"] if hasattr(mha, "ulysses_all_to_all") else [],
+                        "xtuner.v1.module.grouped_linear.moe_group_linear": ["group_gemm"] if hasattr(mgl, "group_gemm") else [],
+                        "xtuner.v1.float8.fsdp_utils": [n for n in ("cast_to_per_block_fp8_with_scales", "tensor_to_per_block_fp8_scales")
+                                                        if hasattr(fu, n)]},
+    )
+    H, I, E, K = 64, 32, 4, 2
+    gate = MoEGate(hidden_size=H, n_routed_experts=E, num_experts_per_tok=K,
+                   router_config=GreedyRouterConfig(scoring_func="softmax", router_scaling_factor=1.0, norm_topk_prob=True))
+    experts = MoEBlock(hidden_size=H, moe_intermediate_size=I, n_routed_experts=E, moe_act_fn_cfg=MoEActFnConfig())
+    keys = {f"gate.{k}": tuple(v.shape) for k, v in gate.state_dict().items()}
+    keys.update({f"experts.{k}": tuple(v.shape) for k, v in experts.state_dict().items()})
+    out["state_dict_shapes_h64_i32_e4_k2"] = keys
+    # fp8 block scales and casts of seeded weights (the stored scales exactly, the e4m3 casts as sha256 of their bytes)
+    g = torch.Generator().manual_seed(5)
+    fp8 = {}
+    for dtype in (torch.float32, torch.bfloat16):
+        w = (torch.randn(3, 256, 384, generator=g) * 2).to(dtype)
+        w[0, :128, :128] = 0
+        s = fu.tensor_to_per_block_fp8_scales(w)
+        fp8[str(dtype)] = dict(scales=s, cast_sha256=[_sha256(fu.cast_to_per_block_fp8_with_scales(w[i], s[i])) for i in range(3)])
+    small = torch.randn(64, 256, generator=g)
+    s_small = torch.rand(2, 1, generator=g) + 0.5
+    fp8["small_cast_sha256"] = _sha256(fu.cast_to_per_block_fp8_with_scales(small, s_small))
+    out["fp8"] = fp8
+    save("reference_seams", out)
+
+
 if __name__ == "__main__":
-    which = sys.argv[1:] or ["noep", "greedy", "noaux", "noaux_bwd", "dispatch", "layer", "variants", "ulysses", "fp8"]
+    which = sys.argv[1:] or ["noep", "greedy", "noaux", "noaux_bwd", "dispatch", "layer", "variants", "ulysses", "fp8", "seams"]
     fns = dict(
         noep=gen_noep_kat,
         greedy=gen_greedy_router,
@@ -462,6 +534,7 @@ if __name__ == "__main__":
         variants=gen_variants,
         ulysses=gen_ulysses,
         fp8=gen_fp8,
+        seams=gen_seams,
     )
     for w in which:
         fns[w]()

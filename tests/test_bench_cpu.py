@@ -97,3 +97,36 @@ def test_reference_arm_prints_contract_line():
     r2 = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2"], capture_output=True,
                         text=True, timeout=120, cwd=ROOT, env=env)
     assert r2.returncode == 0 and r2.stdout.strip() == ""
+
+
+def test_dump_outputs_budget_and_fixed_sample(tmp_path, monkeypatch):
+    """``--dump-outputs``: float32 files, the whole set within the byte budget, arrays above their share sampled at the
+    same positions on every call (two builds dumped with the same arguments compare element for element)."""
+    import numpy as np
+    import torch
+
+    import bench
+
+    monkeypatch.setattr(bench, "DUMP_BYTES", 3 * 4 * 1000)  # three arrays: 1000 elements each at most
+    g = torch.Generator().manual_seed(0)
+    arrays = {"loss": torch.tensor(2.5), "small": torch.randn(10, 20, generator=g).to(torch.bfloat16),
+              "big": torch.randn(300, 70, generator=g)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    total = 0
+    for name, t in arrays.items():
+        a, b = np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy")
+        assert a.dtype == np.float32 and np.array_equal(a, b)
+        total += a.nbytes
+        if t.numel() <= 1000:
+            assert a.shape == tuple(t.shape) and np.array_equal(a, t.float().numpy())
+        else:
+            assert a.shape == (1000,) and np.isin(a, t.numpy().reshape(-1)).all()
+    assert total <= bench.DUMP_BYTES
+
+
+def test_bench_rejects_zero_steps_and_dump_of_the_cpu_arm():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True, timeout=120,
+                           cwd=ROOT)
+        assert r.returncode == 2 and "error" in r.stderr, (extra, r.stderr[-500:])

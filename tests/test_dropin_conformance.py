@@ -1,24 +1,19 @@
-"""Drop-in conformance (CPU, only where /root/reference is mounted — skipped on the GPU box): the host-side mirror
-must expose the reference's seams with the same names, keyword arguments and result keys (SURVEY.md §8b)."""
+"""Drop-in conformance (CPU): the host-side mirror must expose the reference's seams with the same names, keyword arguments
+and result keys (SURVEY.md §8b).  What the reference exposes is stored in ``tests/golden/reference_seams.pt``, read from the
+reference's own classes by ``tests/golden/make_golden.py seams``."""
 import inspect
 import os
 import sys
+import types
 
 import pytest
 
-HERE = os.path.dirname(os.path.abspath(__file__))
-sys.path.insert(0, os.path.join(HERE, "golden"))
-import ref_shim  # noqa: E402
-
-pytestmark = pytest.mark.skipif(not ref_shim.reference_available(), reason="reference tree not mounted")
+from tests.conftest import load_golden
 
 
 @pytest.fixture(scope="module")
 def ref():
-    ref_shim.import_reference()
-    import xtuner.v1  # noqa: F401
-
-    return sys.modules["xtuner.v1"]
+    return load_golden("reference_seams")
 
 
 def _params(fn):
@@ -26,83 +21,74 @@ def _params(fn):
 
 
 def test_dispatcher_methods_match_generic_dispatcher(ref):
-    from xtuner.v1.module.dispatcher.base import GenericDispatcher, NaiveDispatcher
-
     from xtuner_b200.dispatcher import FusedDispatcher
 
-    abstract = sorted(GenericDispatcher.__abstractmethods__)
+    abstract = ref["dispatcher_abstract"]
     assert abstract == ["combine", "combine_postprocess", "combine_preprocess", "dispatch", "dispatch_postprocess", "dispatch_preprocess"]
     for name in abstract:
-        ours, theirs = getattr(FusedDispatcher, name), getattr(NaiveDispatcher, name)
-        op, tp = _params(ours), _params(theirs)
+        op, tp = _params(getattr(FusedDispatcher, name)), ref["dispatcher_params"][name]
         assert [n for n, _, _ in op] == [n for n, _, _ in tp], (name, op, tp)
         assert all(k == inspect.Parameter.KEYWORD_ONLY for _, k, _ in op), f"{name}: keyword-only like the reference"
     # constructor keywords accepted by build_dispatcher (dispatcher/__init__.py:30-96) for the ep=1 case
     ctor = [n for n, _, _ in _params(FusedDispatcher.__init__)]
     for kw in ("n_routed_experts", "process_group", "training_dtype", "generate_dtype"):
-        assert kw in ctor
+        assert kw in ctor and kw in [n for n, _, _ in ref["dispatcher_init"]]
 
 
 def test_op_protocol_signatures(ref):
-    from xtuner.v1.ops.moe.protocol import GroupGemmProtocol, MoePermuteProtocol, MoeUnpermuteProtocol
-
     from xtuner_b200 import ops
 
     def names(fn):
         return [n for n, p in inspect.signature(fn).parameters.items() if n != "self" and p.kind != inspect.Parameter.KEYWORD_ONLY]
 
-    assert names(ops.group_gemm) == names(GroupGemmProtocol.__call__)
-    assert names(ops.permute) == names(MoePermuteProtocol.__call__)
-    assert names(ops.unpermute) == names(MoeUnpermuteProtocol.__call__)
+    want = ref["protocol_positional"]
+    assert names(ops.group_gemm) == want["group_gemm"]
+    assert names(ops.permute) == want["permute"]
+    assert names(ops.unpermute) == want["unpermute"]
 
 
 def test_router_results_keys_and_ctor(ref):
-    from xtuner.v1.module.router.greedy import GreedyRouter as RefGreedy
-    from xtuner.v1.module.router.noaux_router import NoAuxRouter as RefNoAux
-    from xtuner.v1.module.router.protocol import RouterResults as RefResults
-
     from xtuner_b200.router import GreedyRouter, NoAuxRouter, RouterResults
 
-    assert set(RouterResults.__annotations__) == set(RefResults.__annotations__)
-    assert [n for n, _, _ in _params(GreedyRouter.__init__)] == [n for n, _, _ in _params(RefGreedy.__init__)]
-    assert [n for n, _, _ in _params(NoAuxRouter.__init__)] == [n for n, _, _ in _params(RefNoAux.__init__)]
-    assert [n for n, _, _ in _params(GreedyRouter.forward)] == [n for n, _, _ in _params(RefGreedy.forward)]
+    assert sorted(RouterResults.__annotations__) == ref["router_results_keys"]
+    assert [n for n, _, _ in _params(GreedyRouter.__init__)] == [n for n, _, _ in ref["greedy_router_init"]]
+    assert [n for n, _, _ in _params(NoAuxRouter.__init__)] == [n for n, _, _ in ref["noaux_router_init"]]
+    assert [n for n, _, _ in _params(GreedyRouter.forward)] == [n for n, _, _ in ref["greedy_router_forward"]]
 
 
 def test_ulysses_all_to_all_signature(ref):
-    from xtuner.v1.ops.comm.all_to_all import ulysses_all_to_all as ref_fn
-
     from xtuner_b200.comm import ulysses_all_to_all
 
-    assert list(inspect.signature(ulysses_all_to_all).parameters) == list(inspect.signature(ref_fn).parameters)
+    assert list(inspect.signature(ulysses_all_to_all).parameters) == ref["ulysses_all_to_all"]
 
 
 def test_state_dict_keys_match_reference_modules(ref):
-    ref_shim.apply_cpu_patches()
     import torch
-    from xtuner.v1.module.decoder_layer.moe_decoder_layer import MoEActFnConfig, MoEBlock, MoEGate
-    from xtuner.v1.module.router.greedy import GreedyRouterConfig
 
     from xtuner_b200.moe import MoELayer
 
     H, I, E, K = 64, 32, 4, 2
-    gate = MoEGate(hidden_size=H, n_routed_experts=E, num_experts_per_tok=K,
-                   router_config=GreedyRouterConfig(scoring_func="softmax", router_scaling_factor=1.0, norm_topk_prob=True))
-    experts = MoEBlock(hidden_size=H, moe_intermediate_size=I, n_routed_experts=E, moe_act_fn_cfg=MoEActFnConfig())
-    ref_keys = {f"gate.{k}": v.shape for k, v in gate.state_dict().items()}
-    ref_keys.update({f"experts.{k}": v.shape for k, v in experts.state_dict().items()})
     ours = MoELayer(hidden_size=H, moe_intermediate_size=I, n_routed_experts=E, num_experts_per_tok=K)
     our_keys = {k: v.shape for k, v in ours.state_dict().items()}
+    ref_keys = {k: torch.Size(v) for k, v in ref["state_dict_shapes_h64_i32_e4_k2"].items()}
     assert our_keys == ref_keys, (our_keys, ref_keys)
     assert all(isinstance(v, torch.Size) for v in our_keys.values())
 
 
-def test_install_ulysses_rebinds_mha_global(ref):
-    import xtuner.v1.module.attention.mha as mha
-
+def test_install_ulysses_rebinds_mha_global(ref, monkeypatch):
+    """``install_ulysses`` rebinds the module global the reference's attention calls; here that module is a stand-in with
+    the global the reference module has."""
     from xtuner_b200 import comm, plugin
 
-    orig = mha.ulysses_all_to_all
+    name = "xtuner.v1.module.attention.mha"
+    assert ref["module_globals"][name] == ["ulysses_all_to_all"]
+    mha = types.ModuleType(name)
+
+    def orig(input, scatter_dim, gather_dim, mesh):  # noqa: A002
+        raise AssertionError("not called")
+
+    mha.ulysses_all_to_all = orig
+    monkeypatch.setitem(sys.modules, name, mha)
     plugin.install_ulysses()
     try:
         assert mha.ulysses_all_to_all is comm.ulysses_all_to_all

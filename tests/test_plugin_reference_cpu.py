@@ -1,21 +1,31 @@
-"""Engine-level drop-in check on CPU (only where /root/reference is mounted): the reference's OWN Qwen3-style MoE
+"""Engine-level drop-in check on CPU: the reference's OWN Qwen3-style MoE
 model (xtuner.v1.model.moe.moe.MoE: embeddings, attention, MoEDecoderLayer, aux losses, lm_head + CE loss) runs a
 forward+backward with this package's plugin classes installed by ``xtuner_b200.plugin.convert_model`` — FusedDispatcher,
 GreedyRouter, permute/unpermute/group_gemm/swiglu autograd wrappers — and must reproduce the unconverted model's loss and
 gradients exactly.  The CUDA kernels cannot run here, so the *raw kernel entry points* (the torch custom ops that call the
 C-ABI) are replaced by oracle-backed stand-ins inside this test; everything above them (autograd formulas, protocol
-plumbing, dtype/shape conventions, what the reference's layer and losses consume) is the shipped code."""
+plumbing, dtype/shape conventions, what the reference's layer and losses consume) is the shipped code.
+
+The engine-level tests run the reference's model code and so run only where a reference tree is given
+(``XTUNER_REFERENCE_ROOT``).  The last two tests need none: they drive ``plugin`` against stand-ins of the reference modules
+it rebinds and compare with what the reference's functions returned (``tests/golden/reference_seams.pt``)."""
+import hashlib
 import os
 import sys
+import types
 
 import pytest
 import torch
+from torch import nn
+
+from tests.conftest import load_golden
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "golden"))
 import ref_shim  # noqa: E402
 
-pytestmark = pytest.mark.skipif(not ref_shim.reference_available(), reason="reference tree not mounted")
+needs_reference = pytest.mark.skipif(not ref_shim.reference_available(),
+                                     reason="runs the reference's model code: set XTUNER_REFERENCE_ROOT to a reference tree")
 
 
 def _install_cpu_kernel_standins(monkeypatch):
@@ -175,6 +185,7 @@ def _loss_and_grads(model, cfg):
     return {k: v.detach().clone() for k, v in fields.items() if isinstance(v, torch.Tensor) and v.numel() == 1}, grads
 
 
+@needs_reference
 def test_reference_moe_model_with_plugin_matches_unconverted(monkeypatch):
     import torch.distributed as dist
 
@@ -208,6 +219,7 @@ def test_reference_moe_model_with_plugin_matches_unconverted(monkeypatch):
             dist.destroy_process_group()
 
 
+@needs_reference
 def test_reference_moe_model_with_fused_layer_mode(monkeypatch):
     """``convert_model(fused=True)``: the layer's MoE half goes through ``fused.fused_moe_block`` (one autograd node on
     the GPU).  Here that node is an oracle stand-in; what is checked is the glue — which tensors of the reference layer
@@ -291,6 +303,7 @@ def _greedy_route_nocheck(router, logits, top_k, norm_topk_prob=True, router_sca
     return {"logits": logits, "router_weights": rw, "topk_weights": tw, "topk_ids": ids, "topkens_per_expert": tpe}, ids32
 
 
+@needs_reference
 def test_reference_moe_model_with_plugin_through_emulated_cabi(monkeypatch):
     """Same engine-level check, one level lower: the shipped custom-op bodies run and only the C-ABI is emulated."""
     import torch.distributed as dist
@@ -320,6 +333,7 @@ def test_reference_moe_model_with_plugin_through_emulated_cabi(monkeypatch):
             dist.destroy_process_group()
 
 
+@needs_reference
 def test_reference_deepseek_style_model_with_plugin_through_emulated_cabi(monkeypatch):
     """Row a2' at engine level: the reference's MoE model with NoAuxRouterConfig (sigmoid, group-limited top-k, bias) and
     a shared expert, converted by the plugin (NoAuxRouter incl. its new backward, FusedDispatcher, grouped GEMM ops) with
@@ -352,6 +366,7 @@ def test_reference_deepseek_style_model_with_plugin_through_emulated_cabi(monkey
             dist.destroy_process_group()
 
 
+@needs_reference
 def test_reference_moe_model_fused_mode_through_emulated_cabi(monkeypatch):
     """``convert_model(fused=True)`` with the REAL fused node (``fused.FusedMoEBlockFunction``: RMSNorm + gate + route +
     dispatch + experts + combine + residual, and its hand-written backward chain) over the emulated C-ABI, inside the
@@ -385,79 +400,133 @@ def test_reference_moe_model_fused_mode_through_emulated_cabi(monkeypatch):
             dist.destroy_process_group()
 
 
+
+class NaiveDispatcher:
+    """Stand-in for the reference's ep=1 dispatcher: ``convert_model`` recognises it by name and reads these attributes."""
+
+    def __init__(self, n_routed_experts):
+        self._n_routed_experts, self._process_group = n_routed_experts, None
+        self._training_dtype = self._generate_dtype = "bf16"
+
+
+class GreedyRouter(nn.Module):
+    """Stand-in for the reference's GreedyRouter (recognised by name; the attributes ``_convert_router`` copies)."""
+
+    def __init__(self, n_routed_experts, top_k):
+        super().__init__()
+        self.n_routed_experts, self.top_k, self.norm_topk_prob = n_routed_experts, top_k, True
+        self.scoring_func, self.router_scaling_factor = "softmax", 1.0
+
+
+def _standin_moe_model(n_layers=2, E=8, K=2):
+    """Modules laid out like the reference's MoE decoder layers where ``convert_model`` looks: a ``dispatcher`` attribute
+    and ``gate`` (holding ``router``) / ``experts`` sub-modules."""
+    layers = nn.ModuleList()
+    for _ in range(n_layers):
+        layer = nn.Module()
+        layer.dispatcher = NaiveDispatcher(E)
+        layer.gate = nn.Module()
+        layer.gate.router = GreedyRouter(E, K)
+        layer.experts = nn.Module()
+        layers.append(layer)
+    return layers
+
+
+def _standin_module(monkeypatch, ref, name, **globals_):
+    """A stand-in of the reference module ``name`` carrying the globals the reference module has."""
+    assert sorted(ref["module_globals"][name]) == sorted(globals_)
+    mod = types.ModuleType(name)
+    for k, v in globals_.items():
+        setattr(mod, k, v)
+    monkeypatch.setitem(sys.modules, name, mod)
+    return mod
+
+
 def test_convert_model_leaves_unsupported_layers_whole_and_group_gemm_falls_back(monkeypatch):
     """ADVICE r1: (1) a layer whose router has no counterpart must not be half-converted (dispatcher swapped, router not);
     (2) the process-wide ``group_gemm`` rebind must hand inputs our kernels do not cover back to the reference's op."""
-    import torch.distributed as dist
+    from xtuner_b200 import plugin
+    from xtuner_b200.dispatcher import FusedDispatcher
+    from xtuner_b200.router import GreedyRouter as OurGreedyRouter
 
-    if not dist.is_initialized():
-        os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT="29693", RANK="0", WORLD_SIZE="1", LOCAL_RANK="0")
-        dist.init_process_group("gloo", rank=0, world_size=1)
-    try:
-        model, cfg = _build_reference_model(0)
-        from xtuner_b200 import plugin
+    ref = load_golden("reference_seams")
+    calls = []
 
-        layers = [m for m in model.modules() if hasattr(m, "dispatcher")]
+    def ref_group_gemm(x, w, tpe):  # the reference's op as GroupGemmProtocol describes it: one product per expert
+        calls.append(tuple(x.shape))
+        return torch.cat([a @ w[i].T for i, a in enumerate(x.split(tpe.tolist()))])
 
-        class GreedyGroupedRouter(type(layers[0].gate.router)):  # a router class the plugin does not know
-            pass
+    mgl = _standin_module(monkeypatch, ref, "xtuner.v1.module.grouped_linear.moe_group_linear", group_gemm=ref_group_gemm)
+    model = _standin_moe_model()
+    layers = [m for m in model.modules() if hasattr(m, "dispatcher")]
 
-        layers[0].gate.router.__class__ = GreedyGroupedRouter
-        before = [(m.dispatcher, m.gate.router) for m in layers]
-        assert plugin.convert_model(model) == len(layers) - 1
-        assert layers[0].dispatcher is before[0][0] and layers[0].gate.router is before[0][1]
-        assert not hasattr(layers[0], plugin._SAVED)
-        import importlib
+    class GreedyGroupedRouter(GreedyRouter):  # a router class the plugin does not know
+        pass
 
-        mgl = importlib.import_module("xtuner.v1.module.grouped_linear.moe_group_linear")
-        original = getattr(mgl, plugin._SAVED)
-        x = torch.randn(6, 64).to(torch.bfloat16)  # CPU, width 64: not eligible -> the reference's own op answers
-        w = torch.randn(2, 32, 64).to(torch.bfloat16)
-        tpe = torch.tensor([2, 4])
-        assert torch.equal(mgl.group_gemm(x, w, tpe), original(x, w, tpe))
-        plugin.restore_model(model)
-        assert mgl.group_gemm is original
-    finally:
-        if dist.is_initialized():
-            dist.destroy_process_group()
+    layers[0].gate.router.__class__ = GreedyGroupedRouter
+    before = [(m.dispatcher, m.gate.router) for m in layers]
+    assert plugin.convert_model(model) == len(layers) - 1
+    assert layers[0].dispatcher is before[0][0] and layers[0].gate.router is before[0][1]
+    assert not hasattr(layers[0], plugin._SAVED)
+    assert isinstance(layers[1].dispatcher, FusedDispatcher) and isinstance(layers[1].gate.router, OurGreedyRouter)
+    original = getattr(mgl, plugin._SAVED)
+    assert original is ref_group_gemm
+    x = torch.randn(6, 64).to(torch.bfloat16)  # CPU, width 64: not eligible -> the reference's own op answers
+    w = torch.randn(2, 32, 64).to(torch.bfloat16)
+    tpe = torch.tensor([2, 4])
+    assert torch.equal(mgl.group_gemm(x, w, tpe), original(x, w, tpe))
+    assert calls == [(6, 64), (6, 64)]
+    plugin.restore_model(model)
+    assert mgl.group_gemm is original
+    assert layers[1].dispatcher is before[1][0] and layers[1].gate.router is before[1][1]
 
 
 def test_fp8_cast_rebind_matches_the_reference_functions(monkeypatch):
     """``plugin.install_fp8_cast()``: the reference's ``cast_to_per_block_fp8_with_scales`` / ``tensor_to_per_block_fp8_scales``
     (float8/fsdp_utils.py:75-116,196-223 — what ``fsdp_pre_all_gather`` calls on the local shard) routed through the shipped
     wrappers (``ops.fp8_block_cast`` / ``ops.fp8_block_scales``: shape checks, buffer allocation, argument order) over the
-    host-memory emulation of the C-ABI must return the reference's own bits; shapes the kernels do not take (shard rows
-    % 128 == 64, fewer than 128 rows) must stay on the reference's code."""
-    import importlib
-
+    host-memory emulation of the C-ABI must return the reference's own bits (its scales, and the sha256 of its casts, as
+    stored from the reference); shapes the kernels do not take (shard rows % 128 == 64, fewer than 128 rows) must stay on
+    the reference's code."""
     from xtuner_b200 import plugin
 
-    ref_shim.apply_cpu_patches()  # stubs + /root/reference on the path
-    fu = importlib.import_module("xtuner.v1.float8.fsdp_utils")
+    ref = load_golden("reference_seams")
+    want = ref["fp8"]
+    fallback = []
+
+    def ref_cast(tensor, scales, block_size=128, float8_dtype=torch.float8_e4m3fn):
+        fallback.append("cast")
+        return torch.zeros(tensor.shape, dtype=float8_dtype)
+
+    def ref_scales(tensor, reduce_mesh=None, float8_dtype=torch.float8_e4m3fn, block_size=128):
+        fallback.append("scales")
+        return torch.ones(1)
+
+    fu = _standin_module(monkeypatch, ref, "xtuner.v1.float8.fsdp_utils", cast_to_per_block_fp8_with_scales=ref_cast,
+                         tensor_to_per_block_fp8_scales=ref_scales)
     lib = _install_emulated_cabi(monkeypatch)
     monkeypatch.setattr(plugin, "_on_device", lambda t: True)  # host tensors: the eligibility predicate's only device question
-    ref_cast, ref_scales = fu.cast_to_per_block_fp8_with_scales, fu.tensor_to_per_block_fp8_scales
     plugin.install_fp8_cast()
     try:
-        g = torch.Generator().manual_seed(5)
+        g = torch.Generator().manual_seed(5)  # the inputs the stored reference results were computed from
         for dtype in (torch.float32, torch.bfloat16):
             w = (torch.randn(3, 256, 384, generator=g) * 2).to(dtype)
             w[0, :128, :128] = 0  # an all-zero block: scale = EPS / 448
-            want_s = ref_scales(w)
+            want_s = want[str(dtype)]["scales"]
             got_s = fu.tensor_to_per_block_fp8_scales(w)
             assert torch.equal(got_s, want_s) and got_s.shape == (3, 2, 3)
             for i in range(3):
-                want = ref_cast(w[i], want_s[i])
                 got = fu.cast_to_per_block_fp8_with_scales(w[i], want_s[i])
-                assert got.dtype == torch.float8_e4m3fn and torch.equal(got.view(torch.uint8), want.view(torch.uint8))
+                assert got.dtype == torch.float8_e4m3fn
+                assert hashlib.sha256(got.view(torch.uint8).numpy().tobytes()).hexdigest() == want[str(dtype)]["cast_sha256"][i]
         n_ours = len(lib.calls)
         assert lib.calls.count("xtb_fp8_block_cast") == 6 and lib.calls.count("xtb_fp8_block_scales") == 2
+        assert fallback == []
         # shapes outside the kernels' domain stay on the reference path (no library call)
         small = torch.randn(64, 256, generator=g)
         s_small = torch.rand(2, 1, generator=g) + 0.5
-        assert torch.equal(fu.cast_to_per_block_fp8_with_scales(small, s_small).view(torch.uint8), ref_cast(small, s_small).view(torch.uint8))
-        assert len(lib.calls) == n_ours
+        fu.cast_to_per_block_fp8_with_scales(small, s_small)
+        assert fallback == ["cast"] and len(lib.calls) == n_ours
     finally:
         plugin.uninstall_fp8_cast()
     assert fu.cast_to_per_block_fp8_with_scales is ref_cast and fu.tensor_to_per_block_fp8_scales is ref_scales
-
